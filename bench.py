@@ -15,7 +15,8 @@ buffers: upload of the log and of P/Q from pinned memory, one epoch, download of
 of SURVEY.md 8(d): 6*d*4 + 12 = 1548 B per triplet at d = 64.  `cpu_baseline` / `--impl
 reference` time the oracle's port of the reference's numpy loop (the reference ships that loop
 commented out and has nothing to compile, see DESIGN.md) on the host cores.
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0).  `--dump-outputs DIR` also writes the factor tables the last timed step left (see
+dump_tables); the inputs are seeded, so runs with the same arguments start from the same log and tables.
 """
 import argparse
 import json
@@ -83,6 +84,25 @@ def peaks():
         j = json.load(open(p))
         return float(j["hbm_gbs"]), float(j.get("bf16_tflops", 1551.4)), "measured"
     return 6650.0, 1590.0, "fallback"
+
+
+DUMP_TABLE_BYTES = 24 << 20     # --dump-outputs: at most this much of each factor table
+
+
+def dump_tables(out_dir, P, Q):
+    """--dump-outputs: the factor tables the timed steps left, i.e. what yue_get_factors hands a caller of the epoch, as
+    out_dir/P.npy and out_dir/Q.npy in float32.  A table larger than DUMP_TABLE_BYTES is cut to a fixed sample of its rows
+    (seeded, the same rows for the same shape, kept in row order), so that two builds can be compared row for row.
+    The Hogwild epoch is not reproducible (warps read rows while others add to them, in an order the hardware picks), so
+    two runs of ONE build differ too, although their inputs are byte-identical.  Measured on a B200 at config C2: one
+    epoch from the same tables already differs by 2 % of the table norm (median row 0.1 % in P, 2 % in Q); after
+    3 warm-up + 10 timed steps the median row differs by 0.2 % in P and 1.4 % in Q, the worst by 13 % and 26 %."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("P", P), ("Q", Q)):
+        k = min(len(t), DUMP_TABLE_BYTES // (4 * t.shape[1]))
+        if k < len(t):
+            t = t[np.sort(np.random.default_rng(SEED).choice(len(t), k, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(t, dtype=np.float32))
 
 
 class ClockSampler:
@@ -191,6 +211,8 @@ def run_reference(args):
     for w in range(args.warmup):
         cpu_epoch(sample, w)
     t = sum(cpu_epoch(sample, args.warmup + k) for k in range(args.steps))
+    if args.dump_outputs:
+        dump_tables(args.dump_outputs, sample["P"], sample["Q"])
     value = sample["T"] * args.steps / t
     desc = "%d-triplet user-strided sample of the workload per step, oracle port of BPR.py:31-62" % sample["T"]
     emit(json.dumps({
@@ -329,6 +351,8 @@ def run_native(args):
     barrier()
     clk = clocks.stop() if rank == 0 else None
     launches = eng.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_tables(args.dump_outputs, *eng.get_factors())
     ms = allmax(ms)
     value = T * world * args.steps / (ms * 1e-3)
     achieved = bpt * T / (k_ms * 1e-3) / 1e9
@@ -878,7 +902,11 @@ def main():
     ap.add_argument("--no-apr", action="store_true")
     ap.add_argument("--no-wrmf", action="store_true")
     ap.add_argument("--rank-users", type=int, default=1_000_000)   # config C4: 1 M users
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the factor tables they left (rank 0's) to DIR as float32 .npy (see dump_tables)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and not args.small:
         args.warmup = 3
     quiet_stdout()

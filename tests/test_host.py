@@ -151,3 +151,28 @@ def test_bench_clock_sampler_windows_on_the_timed_region():
     out = sampler([(-1.0, idle), (-0.5, busy)], mark_at=-0.05).stop()
     assert out["samples"] == 2 and out["window"].startswith("warm-up + timed region")
     assert bench.ClockSampler(0).stop()["reasons"] == ["nvidia-smi unavailable"]
+
+
+def test_bench_dump_tables_keeps_small_tables_and_samples_large_ones_by_a_fixed_seed(tmp_path):
+    """bench.py --dump-outputs: float32 .npy per table, a table within the budget whole, a larger one as the same sorted
+    sample of its rows on every call, and both files together within 2 x the per-table budget."""
+    import importlib.util
+    import os
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_for_test", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    bench.DUMP_TABLE_BYTES = 64 * 4 * 1000                       # 1000 rows of d = 64
+    P = np.arange(5000 * 64, dtype=np.float64).reshape(5000, 64)
+    Q = np.random.default_rng(1).random((700, 64), dtype=np.float32)
+    got = []
+    for run in ("a", "b"):
+        bench.dump_tables(str(tmp_path / run), P, Q)
+        got.append({n: np.load(str(tmp_path / run / (n + ".npy"))) for n in ("P", "Q")})
+    p, q = got[0]["P"], got[0]["Q"]
+    assert p.dtype == np.float32 and q.dtype == np.float32 and p.shape == (1000, 64)
+    rows = p[:, 0].astype(np.int64) // 64
+    assert np.all(np.diff(rows) > 0) and np.array_equal(p, P[rows].astype(np.float32))
+    assert np.array_equal(q, Q)
+    assert np.array_equal(got[1]["P"], p) and np.array_equal(got[1]["Q"], q)
+    assert sum(os.path.getsize(str(tmp_path / "a" / f)) for f in os.listdir(str(tmp_path / "a"))) <= 2 * bench.DUMP_TABLE_BYTES + 512

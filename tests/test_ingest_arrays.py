@@ -16,6 +16,7 @@ from yue_b200.host.config import Config, LineConfig
 from yue_b200.host.fileio import DataSplit
 from yue_b200.host.measure import Measure
 
+REF = os.environ.get("YUE_REFERENCE", "")          # a checkout of 0411tony/Yue: when set, one more comparison
 COLUMNS = {"user": 1, "track": 2, "artist": 3, "time": 0}          # record.setup of config/BPR.conf: -columns user:1,track:2,artist:3,time:0
 
 
@@ -180,9 +181,9 @@ def test_cv_folds_equal_the_reference_split_numbered_fold_by_fold(golden_dir, tm
 
 
 @pytest.mark.parametrize("ev", ["-target track -ap 0.2 -cold 3", "-target track -ap 0.2 -sample", "-target track -ap 0.2 -cold 5 -sample"])
-def test_cold_and_sample_edit_the_test_csr_like_the_dict_form(golden_dir, ev):
+def test_cold_and_sample_edit_the_test_csr_like_the_dict_form(golden_dir, tmp_path, ev):
     """base/recommender.py:22-49 (-cold t, -sample) on the CSR form of the test set (ingest.filter_test_rows) against the
-    dict form the Recommender base class edits -- and, in the build container, against the REFERENCE's own base class."""
+    dict form the Recommender base class edits -- and, given a checkout of the reference, against its own base class."""
     from yue_b200.host.recommender import Recommender
     g = json.load(open(os.path.join(golden_dir, "record_small.json")))
     train = [e for e, h in zip(g["events"], g["held"]) if not h]
@@ -193,17 +194,17 @@ def test_cold_and_sample_edit_the_test_csr_like_the_dict_form(golden_dir, ev):
     with redirect_stdout(io.StringIO()):
         ref = Recommender(Config(values=vals), train, test)
     want = {u: sorted(t) for u, t in ref.data.testSet.items()}
-    if os.path.isdir("/root/reference"):                         # the reference's own base class says the same
+    if os.path.isdir(REF):                         # the reference's own base class says the same
         import subprocess
         import sys
-        code = ("import sys, json, io\nfrom contextlib import redirect_stdout\nsys.path.insert(0, '/root/reference')\n"
+        code = ("import sys, json, io\nfrom contextlib import redirect_stdout\nsys.path.insert(0, %r)\n"
                 "from tool.config import Config\nfrom base.recommender import Recommender\n"
                 "g = json.load(open(%r))\ntrain = [e for e, h in zip(g['events'], g['held']) if not h]\n"
                 "test = [e for e, h in zip(g['events'], g['held']) if h]\nopen(%r, 'w').write(%r)\n"
                 "with redirect_stdout(io.StringIO()):\n    r = Recommender(Config(%r), train, test)\n"
                 "print(json.dumps({u: sorted(t) for u, t in r.data.testSet.items()}))\n"
-                % (os.path.join(golden_dir, "record_small.json"), "/tmp/_yue_cold.conf",
-                   "\n".join(k + "=" + v for k, v in vals.items()), "/tmp/_yue_cold.conf"))
+                % (REF, os.path.join(golden_dir, "record_small.json"), str(tmp_path / "c.conf"),
+                   "\n".join(k + "=" + v for k, v in vals.items()), str(tmp_path / "c.conf")))
         res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=120)
         assert res.returncode == 0, res.stderr
         assert json.loads(res.stdout.strip().splitlines()[-1]) == want

@@ -10,12 +10,16 @@ Tolerances (float32 kernel against the float64 restatement): the loss of a step 
 step (read back from Adam's first moment, m_1 = 0.1 g) 2e-4 of the largest row gradient, per row; the propagated tables
 1e-5 per row.  After several Adam steps a table entry whose gradient is rounding noise may differ by a full step (Adam
 divides by |g|), so the tables after a run are compared entry-wise: at least 99.5 % within 2 % of the distance moved."""
+import os
+
 import numpy as np
 import pytest
 
 from oracle import lightgcn_ref as lg
 from oracle import philox
 from yue_b200 import synth
+
+REF = os.environ.get("YUE_REFERENCE", "")          # a checkout of 0411tony/Yue; the shim test skips without one
 
 
 def file_order(log, seed):
@@ -149,12 +153,11 @@ def test_both_ingest_modes_give_the_class_the_same_batches(golden_dir, tmp_path)
     assert names[ua[:20]].tolist() == [b.data.id2name["user"][int(x)] for x in ub[:20]]
 
 
-@pytest.mark.skipif(not __import__("os").path.isdir("/root/reference"), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the Yue reference: set YUE_REFERENCE to its directory")
 def test_dropin_shim_on_top_of_the_reference_tree(golden_dir, tmp_path):
     """dropin/recommender/advanced/LightGCN.py shadows the reference's module (TF-1, unimportable base), derives from the
     REFERENCE's own base.IterativeRecommender and Record (under -byTime: the reference's own time split), and drives the
     engine with the calls INTEGRATION.md lists -- checked with a recording engine in place of the CUDA one."""
-    import os
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -166,7 +169,7 @@ def test_dropin_shim_on_top_of_the_reference_tree(golden_dir, tmp_path):
 import io, json, sys
 import numpy as np
 from contextlib import redirect_stdout
-sys.path[:0] = [%(dropin)r, "/root/reference", %(root)r]
+sys.path[:0] = [%(dropin)r, %(ref)r, %(root)r]
 from tool.config import Config
 from recommender.advanced.LightGCN import LightGCN
 import base.IterativeRecommender as ref_base
@@ -198,7 +201,7 @@ assert calls[2] == ("epoch", 128, 0.002, 0.001, 11, 0, 3) and calls[3] == ("epoc
 assert calls[4] == ("finalize", 3) and m.loss == 3.0
 assert m.multi_item_embeddings.shape == (3, 50) and "training: 2 batch 2 loss: 3.0" in out.getvalue()
 print("shim ok")
-''' % dict(dropin=os.path.join(root, "dropin"), root=root, gold=golden_dir, tmp=str(tmp_path), conf=conf)
+''' % dict(dropin=os.path.join(root, "dropin"), ref=REF, root=root, gold=golden_dir, tmp=str(tmp_path), conf=conf)
     res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
     assert res.returncode == 0 and "shim ok" in res.stdout, res.stdout + res.stderr
 

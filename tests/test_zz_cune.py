@@ -12,6 +12,8 @@ import pytest
 from oracle import cune_ref, philox, record_ref
 from yue_b200.host.config import Config
 
+REF = os.environ.get("YUE_REFERENCE", "")          # a checkout of 0411tony/Yue; the shim test skips without one
+
 
 def _golden_slice(golden_dir):
     g = json.load(open(os.path.join(golden_dir, "record_small.json")))
@@ -375,7 +377,7 @@ def test_cune_kernel_text_at_the_device_warp_width(golden_dir, tmp_path):
         assert loss.value == pytest.approx(float(ref), rel=1e-5 if serial else 1e-3)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs a checkout of the Yue reference: set YUE_REFERENCE to its directory")
 def test_cune_dropin_shim_on_top_of_the_reference_tree(golden_dir, tmp_path):
     """dropin/recommender/advanced/CUNE.py shadows the reference's module (which needs gensim at import), derives from the
     REFERENCE's own base.IterativeRecommender and Record, and with the oracle in place of yue_cune_epoch reproduces the
@@ -387,7 +389,7 @@ def test_cune_dropin_shim_on_top_of_the_reference_tree(golden_dir, tmp_path):
 import io, json, os, sys
 import numpy as np
 from contextlib import redirect_stdout
-sys.path[:0] = [%(dropin)r, "/root/reference", %(root)r]
+sys.path[:0] = [%(dropin)r, %(ref)r, %(root)r]
 from tool.config import Config
 from recommender.advanced.CUNE import CUNE
 import base.IterativeRecommender as ref_base
@@ -429,7 +431,7 @@ with redirect_stdout(io.StringIO()):
 assert np.array_equal(e.ip[1], w["ip_items"])
 assert np.array_equal(m.P, w["P"][-1]) and np.array_equal(m.Q, w["Q"][-1])
 print("OK")
-''' % dict(dropin=os.path.join(root, "dropin"), root=root, gold=golden_dir, tmp=str(tmp_path), conf=_conf(tmp_path))
+''' % dict(dropin=os.path.join(root, "dropin"), ref=REF, root=root, gold=golden_dir, tmp=str(tmp_path), conf=_conf(tmp_path))
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=str(tmp_path))
     assert r.returncode == 0 and "OK" in r.stdout, r.stderr[-2000:]
 
