@@ -281,8 +281,10 @@ def test_blocked_kernel_read_schedule_is_pinned_when_tracks_repeat(engine, d, n)
     the conflict-free test avoids and the quality checks only see statistically.  One warp (the log is far below a second
     warp's share), tiny catalogs (7-40 tracks: repeats in nearly every block), users with 1..70 triplets: the tables must
     equal oracle/bpr_blk_ref.py -- the reference's arithmetic per triplet, rows of block k read before block k-1's changes
-    are added, every change added -- to 1e-4 (a row of a 7-track catalog takes ~600 float32 adds whose rounding depends
-    on the order the atomics land in; measured 4e-6 on P, 2e-5 on Q), the loss to 1e-5; the serial order is 100x further."""
+    are added, every change added -- to 1e-4 (a row of a 7-track catalog takes ~600 float32 adds; the kernel's scores come
+    from the Gram recurrence and the oracle's from a float64 dot, so the roundings differ; measured 4e-6 on P, 2e-5 on Q),
+    the loss to 1e-5; the serial order is 100x further.  At one warp the epoch is deterministic: one lane adds every
+    float in program order, and the same epoch run twice gives the same bits (tests/test_sgd_epoch_schedule_gpu.py)."""
     from oracle import bpr_blk_ref
     m = 60
     rng = np.random.default_rng(d * 100 + n)
