@@ -190,6 +190,31 @@ int yue_gcn_finalize(yue_t* h, int n_layers);
  * V, [m, k] and [n, k] each (NULL = skip), and the number of steps taken since yue_set_factors. */
 int yue_gcn_moments(yue_t* h, float* m_users, float* m_tracks, float* v_users, float* v_tracks, int64_t* steps);
 
+/* BPR as the reference ships it (recommender/cf/BPR.py:65-129, SURVEY.md 3.3; the per-triplet loop of 31-62 is commented out
+ * there): a TF-1 graph trained with AdamOptimizer on sampled mini-batches.  Step s draws `batch` training events uniformly
+ * with replacement (next_batch, 65-81: np.random.randint at 66) and, per event, `negatives` unplayed tracks (uniform
+ * over all n tracks, random.randint rejected against the user's plays, 74-76); loss = sum over the batch x negatives triplets of
+ * softplus(-(U_u.V_i - U_u.V_j)) + reg (l2_loss(U_u) + l2_loss(V_i) + l2_loss(V_j)) with the rows read before the step
+ * (93-115; regU for all three terms); one Adam step (beta 0.9 / 0.999, epsilon 1e-8) on EVERY row of U and V, num.max.iter steps (121-129).
+ * U, V are the handle's factor tables (the graph's truncated_normal(0.005) init is the caller's); yue_set_factors restarts
+ * Adam.  The moments are this path's own (not yue_gcn_*'s).  Sampler: Philox (yue_sample_negatives' stream) with epoch = s,
+ * event = the batch row b: the event is attempt 0 of slot 4095 scaled to [0, T) (e = (r T) >> 32), negative k is slot k with
+ * rejection -- the batch is a pure function of (seed, s).  Needs the whole log on one handle, T < 2^32, negatives <= 4095.
+ * yue_bpr_adam_sample:  check hook (needs the log, not the factors), the batch of step `step`: events_out[batch]
+ *   (indices into the event CSR) and neg_out[batch * negatives] (row-major by batch row).  Replaces next_batch, BPR.py:65-81.
+ * yue_bpr_adam_steps:   steps [step_begin, step_end); loss_out[s - step_begin] = that step's loss (may be NULL), what
+ *   the loop prints.  Replaces the loop of BPR.py:121-129 (the graph's Session.run).  Any split of a step range gives
+ *   the same bits as the whole range; a non-finite loss is YUE_E_NUMERIC.
+ * yue_bpr_adam_apply:   one step on the caller's B triplets (parity hook, no sampler); *loss_out = its loss.
+ * yue_bpr_adam_moments: Adam's first / second moments of U and V ([m, k], [n, k]; NULL = skip) and the steps taken since
+ *   yue_set_factors (checkpointing; tests read the first step's gradient from them: m_1 = 0.1 g). */
+int yue_bpr_adam_sample(yue_t* h, uint64_t seed, int64_t step, int batch, int negatives, int32_t* events_out, int32_t* neg_out);
+int yue_bpr_adam_steps(yue_t* h, int batch, int negatives, double lr, double reg, uint64_t seed, int64_t step_begin,
+                       int64_t step_end, double* loss_out);
+int yue_bpr_adam_apply(yue_t* h, int64_t B, const int32_t* u, const int32_t* i, const int32_t* j, double lr, double reg,
+                       double* loss_out);
+int yue_bpr_adam_moments(yue_t* h, float* m_users, float* m_tracks, float* v_users, float* v_tracks, int64_t* steps);
+
 /* (P*P).sum(), (Q*Q).sum() of BPR.py:59, accumulated in float64. */
 int yue_frob2(yue_t* h, double* p2, double* q2);
 

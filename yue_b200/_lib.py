@@ -113,6 +113,10 @@ SIGNATURES = {
     "yue_gcn_apply": (C.c_int, [_H, C.c_int, C.c_int64, _i32p, _i32p, _i32p, C.c_double, C.c_double, _f64p]),
     "yue_gcn_finalize": (C.c_int, [_H, C.c_int]),
     "yue_gcn_moments": (C.c_int, [_H, _f32p, _f32p, _f32p, _f32p, _i64p]),
+    "yue_bpr_adam_sample": (C.c_int, [_H, C.c_uint64, C.c_int64, C.c_int, C.c_int, _i32p, _i32p]),
+    "yue_bpr_adam_steps": (C.c_int, [_H, C.c_int, C.c_int, C.c_double, C.c_double, C.c_uint64, C.c_int64, C.c_int64, _f64p]),
+    "yue_bpr_adam_apply": (C.c_int, [_H, C.c_int64, _i32p, _i32p, _i32p, C.c_double, C.c_double, _f64p]),
+    "yue_bpr_adam_moments": (C.c_int, [_H, _f32p, _f32p, _f32p, _f32p, _i64p]),
     "yue_frob2": (C.c_int, [_H, _f64p, _f64p]),
     "yue_predict": (C.c_int, [_H, C.c_int64, _f32p]),
     "yue_rank_topn": (C.c_int, [_H, _i32p, C.c_int64, C.c_int, C.c_int, _i32p, _f32p]),

@@ -11,8 +11,8 @@ the reference's base classes provide (``self.data`` = Record, ``self.k``, ``self
   ``dropin/recommender/cf/BPR.py`` (INTEGRATION.md).
 
 What replaces what (reference paths):
-  buildModel   recommender/cf/BPR.py:31-62 -- the per-triplet SGD loop (numpy text; the shipped
-               TF/Adam variant at 83-129 is documented in DESIGN.md and not reproduced)
+  buildModel   recommender/cf/BPR.py:31-62 -- the per-triplet SGD loop (numpy text, the default); with
+               yue.train=adam the shipped TF/Adam training of 65-129 (K10, csrc/bpr_adam.cuh)
   predict      recommender/cf/BPR.py:131-134
   evalRanking  base/IterativeRecommender.py:77-173, with the EXACT masked top-N instead of the
                lossy selection at 107-145 (SURVEY.md R5)
@@ -36,6 +36,9 @@ class GpuBPRMixin(object):
     #: optional config keys understood on top of the reference's (all have defaults)
     #:   yue.device=<int>      CUDA device (default $YUE_DEVICE or 0)
     #:   yue.sgd=hogwild|serial  update schedule (default hogwild; serial = reference order)
+    #:   yue.train=sgd|adam    sgd (default): the per-triplet SGD loop of BPR.py:31-62; adam: what BPR.py:65-129 runs --
+    #:                         truncated_normal(0.005) tables, num.max.iter Adam steps on 512 sampled events x 100
+    #:                         negatives each, the loss and ranking_performance() after every step (one device)
     #:   yue.seed=<int>        sampler seed (default: drawn from `random`, unseeded like the reference)
     #:   yue.ingest=host|device   where the array form of the log (event CSR, play sets, test sets) is built: host =
     #:                         numpy on Record's dicts; device = yue_ingest_events on the numbered events (K0)
@@ -135,7 +138,18 @@ class GpuBPRMixin(object):
         self.n = self.data.getSize(self.recType)
         self.train_size = len(self.data.trainingData)
 
+    #: batch rows and negatives per row of yue.train=adam (BPR.py:65-81)
+    adam_batch, adam_negatives = 512, 100
+
+    def _train_mode(self):
+        train = str(self._opt('yue.train', 'sgd')).strip()
+        if train not in ('sgd', 'adam'):
+            raise ValueError('yue.train must be sgd or adam, not %r' % train)
+        return train
+
     def buildModel(self):
+        if self._train_mode() == 'adam':
+            return self._build_adam()
         print('training...')
         eng = self._push_factors()
         mode = MODE_SERIAL if self._opt('yue.sgd', 'hogwild') == 'serial' else MODE_HOGWILD
@@ -152,6 +166,25 @@ class GpuBPRMixin(object):
             if self.isConverged(iteration):
                 break
         self._pull_factors()
+
+    def _build_adam(self):
+        """BPR.py:93-129: U, V ~ truncated_normal(0.005), then num.max.iter Adam steps on sampled batches, each followed by
+        the tables on the host (self.P, self.Q), the loss and ranking_performance().  No lr schedule, no isConverged."""
+        from .lightgcn import truncated_normal
+        print('training...')
+        devs = self._devices()
+        if len(devs) > 1:
+            print('yue.devices: yue.train=adam trains on device %d alone; ranking uses all devices' % devs[0])
+        self.P = truncated_normal((self.m, self.k), 0.005)
+        self.Q = truncated_normal((self.n, self.k), 0.005)
+        eng = self._push_factors()
+        seed = int(self._opt('yue.seed', random.getrandbits(63)))
+        for step in range(self.maxIter):
+            loss = eng.bpr_adam_steps(self.adam_batch, self.adam_negatives, self.lRate, self.regU, seed, step, step + 1)
+            self.loss = float(loss[0])
+            self._pull_factors()
+            print('iteration:', step + 1, 'loss:', self.loss)
+            self.ranking_performance()
 
     def _sharded_session(self, eng, devs):
         """buildModel over several GPUs.  BPR.py:40-62 with the users dealt out to the devices (user u on devs[u % N], so

@@ -27,6 +27,7 @@
 #include "wrmf_als.cuh"
 #include "cune_sgd.cuh"
 #include "lightgcn.cuh"
+#include "bpr_adam.cuh"
 
 using namespace yue;
 
@@ -237,6 +238,15 @@ struct yue_handle {
     std::vector<int64_t> h_it_indptr;
     int64_t gcn_n_chunk = 0, gcn_n_seg = 0, gcn_t = 0;
     uint32_t gcn_stamp_base = 0;
+
+    // BPR's shipped Adam training (K10): Adam's moments (separate from K9's), the step counter, the per-step scratch
+    DevBuf<float> ba_am, ba_av, ba_trip_c, ba_trip_loss, ba_ucopy, ba_ugrad, ba_row_c;
+    DevBuf<int32_t> ba_fix, ba_row_u, ba_row_i, ba_row_e, ba_trip_j, ba_slot_row, ba_slot_pos, ba_list, ba_sorted, ba_cnt, ba_row_base, ba_row_size;
+    DevBuf<uint32_t> ba_stamp;
+    DevBuf<unsigned> ba_bump;
+    DevBuf<double> ba_row_loss, ba_loss;
+    int64_t ba_t = 0;
+    uint32_t ba_tag = 0;
 
     ncclComm_t comm = nullptr;
     int nranks = 1, rank = 0;
@@ -459,6 +469,9 @@ int yue_destroy(yue_t* h) {
     h->gcn_segs.release(); h->gcn_chunks.release(); h->gcn_arrived.release(); h->gcn_phase_ns.release();
     for (auto* b : {&h->gcn_E[0], &h->gcn_E[1], &h->gcn_E[2], &h->gcn_E[3], &h->gcn_rinv, &h->gcn_D[0], &h->gcn_D[1], &h->gcn_am, &h->gcn_av, &h->gcn_slot_grad, &h->gcn_NB, &h->gcn_trip_loss, &h->gcn_varP, &h->gcn_varQ, &h->gcn_partial}) b->release();
     h->gcn_stamp.release(); h->gcn_loss.release();
+    for (auto* b : {&h->ba_am, &h->ba_av, &h->ba_trip_c, &h->ba_trip_loss, &h->ba_ucopy, &h->ba_ugrad, &h->ba_row_c}) b->release();
+    for (auto* b : {&h->ba_fix, &h->ba_row_u, &h->ba_row_i, &h->ba_row_e, &h->ba_trip_j, &h->ba_slot_row, &h->ba_slot_pos, &h->ba_list, &h->ba_sorted, &h->ba_cnt, &h->ba_row_base, &h->ba_row_size}) b->release();
+    h->ba_stamp.release(); h->ba_bump.release(); h->ba_row_loss.release(); h->ba_loss.release();
     h->hot_base.release(); h->Qown.release(); h->Qsum.release();
     for (void* p : h->ipc_opened) cudaIpcCloseMemHandle(p);
     if (h->ev_pack) cudaEventDestroy(h->ev_pack);
@@ -845,6 +858,7 @@ int yue_set_factors(yue_t* h, int k, const float* P, const float* Q) {
     CK(cudaStreamSynchronize(h->stream));
     h->have_factors = true;
     h->gcn_t = 0; h->gcn_final = false;         // new variables: Adam starts over
+    h->ba_t = 0;                                // (K9's and K10's Adam alike)
     h->have_snap = false;
     h->exchange_pending = false;
     h->hot_shared = false;                     // new tables: the owners' rows no longer describe them
@@ -1565,6 +1579,186 @@ int yue_gcn_moments(yue_t* h, float* m_users, float* m_tracks, float* v_users, f
     struct { float* dst; const float* src; int64_t rows; } parts[4] = {
         {m_users, h->gcn_am.p, h->m}, {m_tracks, have ? h->gcn_am.p + (size_t)h->m * ld : nullptr, h->n},
         {v_users, h->gcn_av.p, h->m}, {v_tracks, have ? h->gcn_av.p + (size_t)h->m * ld : nullptr, h->n}};
+    for (auto& x : parts) {
+        if (!x.dst || x.rows == 0) continue;
+        if (!have) { std::memset(x.dst, 0, (size_t)x.rows * k * sizeof(float)); continue; }
+        CK(cudaMemcpy2DAsync(x.dst, k * sizeof(float), x.src, ld * sizeof(float), k * sizeof(float), (size_t)x.rows, cudaMemcpyDeviceToHost, h->stream));
+    }
+    CK(cudaStreamSynchronize(h->stream));
+    return YUE_OK;
+}
+
+// ---- K10: BPR's shipped Adam training (bpr_adam.cuh) ------------------------------------------------------------------
+static int bpr_adam_check(yue_t* h, int64_t batch, int64_t negatives, bool need_factors = true) {
+    REQUIRE(h && h->have_log, YUE_E_STATE, "interactions not set");
+    REQUIRE(h->have_factors || !need_factors, YUE_E_STATE, "factors not set");
+    REQUIRE(batch >= 1 && batch <= (1 << 16), YUE_E_ARG, "batch must be in 1..65536");
+    REQUIRE(negatives >= 1 && negatives <= (int64_t)kBprAdamPosSlot, YUE_E_ARG, "negatives must be in 1..4095 (slot 4095 draws the positive)");
+    REQUIRE(batch * negatives <= (1 << 24), YUE_E_ARG, "batch x negatives must be at most 2^24 triplets");
+    REQUIRE(h->user_begin == 0 && h->event_base == 0 && !h->have_ev_delta, YUE_E_UNSUPPORTED, "Adam training needs the whole log on one handle");
+    REQUIRE(!h->hot_shared, YUE_E_UNSUPPORTED, "the hot rows are shared (yue_hot_unshare first)");
+    REQUIRE(h->m + h->n < ((int64_t)1 << 31), YUE_E_UNSUPPORTED, "more than 2^31 table rows");
+    CK(cudaSetDevice(h->device));
+    return need_factors ? q_rowmajor(h) : YUE_OK;
+}
+
+// scratch for `rows` x `negatives`; Adam's moments (zero when the step counter is)
+static int bpr_adam_buffers(yue_t* h, int64_t rows, int64_t negatives) {
+    const size_t M = (size_t)(h->m + h->n), ld = (size_t)h->ld, N = (size_t)(rows * negatives), S = 2 * (size_t)rows + N;
+    cudaStream_t st = h->stream;
+    const bool fresh = h->ba_am.n < M * ld || h->ba_av.n < M * ld || h->ba_t == 0;
+    CK(h->ba_am.resize(M * ld)); CK(h->ba_av.resize(M * ld));
+    if (fresh) {
+        CK(cudaMemsetAsync(h->ba_am.p, 0, M * ld * sizeof(float), st)); CK(cudaMemsetAsync(h->ba_av.p, 0, M * ld * sizeof(float), st));
+        h->ba_t = 0;
+    }
+    if (h->ba_stamp.n < M || h->ba_tag > 0xF0000000u) {
+        CK(h->ba_stamp.resize(M)); CK(h->ba_cnt.resize(M));
+        CK(cudaMemsetAsync(h->ba_stamp.p, 0, M * sizeof(uint32_t), st)); CK(cudaMemsetAsync(h->ba_cnt.p, 0, M * sizeof(int32_t), st));
+        h->ba_tag = 0;
+    }
+    CK(h->ba_row_base.resize(M)); CK(h->ba_row_size.resize(M));
+    CK(h->ba_row_u.resize((size_t)rows)); CK(h->ba_row_i.resize((size_t)rows)); CK(h->ba_row_e.resize((size_t)rows));
+    CK(h->ba_row_c.resize((size_t)rows)); CK(h->ba_row_loss.resize((size_t)rows));
+    CK(h->ba_ucopy.resize((size_t)rows * ld)); CK(h->ba_ugrad.resize((size_t)rows * ld));
+    CK(h->ba_trip_j.resize(N)); CK(h->ba_trip_c.resize(N)); CK(h->ba_trip_loss.resize(N));
+    CK(h->ba_slot_row.resize(S)); CK(h->ba_slot_pos.resize(S)); CK(h->ba_list.resize(S)); CK(h->ba_sorted.resize(S));
+    CK(h->ba_bump.resize(1));
+    return YUE_OK;
+}
+
+static BprAdamParams bpr_adam_params(yue_t* h, int64_t rows, int64_t negatives, double reg) {
+    BprAdamParams p{};
+    p.m = h->m; p.n = h->n; p.T = h->T; p.ld = h->ld; p.B = (int)rows; p.K = (int)negatives;
+    p.ev_user = h->ev_user.p; p.ev_items = h->ev_items.p; p.hot_items = h->hot_items.p;
+    p.uq_indptr = h->uq_indptr.p; p.uq_items = h->uq_items.p;
+    p.P = h->P.p; p.Q = h->Q.p; p.am = h->ba_am.p; p.av = h->ba_av.p;
+    p.reg = (float)reg;
+    p.row_u = h->ba_row_u.p; p.row_i = h->ba_row_i.p; p.row_e = h->ba_row_e.p;
+    p.trip_j = h->ba_trip_j.p; p.trip_c = h->ba_trip_c.p; p.trip_loss = h->ba_trip_loss.p;
+    p.ucopy = h->ba_ucopy.p; p.ugrad = h->ba_ugrad.p; p.row_c = h->ba_row_c.p; p.row_loss = h->ba_row_loss.p;
+    p.slot_row = h->ba_slot_row.p; p.slot_pos = h->ba_slot_pos.p; p.list = h->ba_list.p; p.sorted = h->ba_sorted.p;
+    p.cnt = h->ba_cnt.p; p.row_base = h->ba_row_base.p; p.row_size = h->ba_row_size.p; p.stamp = h->ba_stamp.p; p.bump = h->ba_bump.p;
+    return p;
+}
+
+template <int G, int NC>
+static void bpr_adam_launch_groups(yue_t* h, const BprAdamParams& p) {
+    constexpr int GPB = kBprAdamThreads / G;
+    const int64_t N = (int64_t)p.B * p.K;
+    const int cap = h->sm_count * 8;
+    bpr_adam_triplet_kernel<G, NC><<<(unsigned)std::max<int64_t>(1, std::min<int64_t>((N + GPB - 1) / GPB, cap)), kBprAdamThreads, 0, h->stream>>>(p);
+    bpr_adam_row_kernel<G, NC><<<(unsigned)std::max<int64_t>(1, std::min<int64_t>((p.B + GPB - 1) / GPB, cap)), kBprAdamThreads, 0, h->stream>>>(p);
+}
+
+// one step: six launches on the handle's stream; the loss stays on the device (p.loss_out)
+static int bpr_adam_step(yue_t* h, BprAdamParams& p, double lr) {
+    const int64_t t = h->ba_t + 1;
+    p.lr_t = (float)(lr * std::sqrt(1.0 - std::pow(0.999, (double)t)) / (1.0 - std::pow(0.9, (double)t)));
+    p.tag = ++h->ba_tag;
+    if (h->ld <= 16) bpr_adam_launch_groups<4, 1>(h, p);
+    else if (h->ld <= 32) bpr_adam_launch_groups<8, 1>(h, p);
+    else if (h->ld <= 64) bpr_adam_launch_groups<16, 1>(h, p);
+    else if (h->ld <= 128) bpr_adam_launch_groups<32, 1>(h, p);
+    else bpr_adam_launch_groups<32, 2>(h, p);
+    const int64_t S = 2 * (int64_t)p.B + (int64_t)p.B * p.K;
+    const unsigned sg = (unsigned)std::max<int64_t>(1, std::min<int64_t>((S + 255) / 256, (int64_t)h->sm_count * 8));
+    bpr_adam_alloc_kernel<<<sg, 256, 0, h->stream>>>(p);
+    bpr_adam_scatter_kernel<<<sg, 256, 0, h->stream>>>(p);
+    bpr_adam_rank_kernel<<<sg, 256, 0, h->stream>>>(p);
+    // the dense pass: one float4 per thread, as many CTAs as keep the SMs' load queues full
+    const int64_t f4 = (h->m + h->n) * (h->ld / 4);
+    const unsigned ug = (unsigned)std::max<int64_t>(1, std::min<int64_t>((f4 + kBprAdamThreads - 1) / kBprAdamThreads, (int64_t)h->sm_count * 32));
+    bpr_adam_update_kernel<<<ug, kBprAdamThreads, 0, h->stream>>>(p);
+    h->launches += 6;
+    CK(cudaGetLastError());
+    h->ba_t = t;
+    return YUE_OK;
+}
+
+// copies `steps` losses back, marks the derived copies of Q stale, refuses a non-finite loss
+static int bpr_adam_finish(yue_t* h, int64_t steps, double* loss_out) {
+    h->ilv_current = false; h->tc.q_dirty = true;
+    std::vector<double> loss((size_t)steps);
+    CK(cudaMemcpyAsync(loss.data(), h->ba_loss.p, steps * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    bool finite = true;
+    for (int64_t s = 0; s < steps; ++s) { if (loss_out) loss_out[s] = loss[s]; finite = finite && std::isfinite(loss[s]); }
+    if (!finite) return fail(h, YUE_E_NUMERIC, "Loss = NaN or Infinity: current settings does not fit the recommender!");
+    return YUE_OK;
+}
+
+int yue_bpr_adam_sample(yue_t* h, uint64_t seed, int64_t step, int batch, int negatives, int32_t* events_out, int32_t* neg_out) {
+    if (int rc = bpr_adam_check(h, batch, negatives, false)) return rc;
+    REQUIRE(events_out && neg_out, YUE_E_ARG, "null output");
+    REQUIRE(step >= 0 && step <= (int64_t)UINT32_MAX, YUE_E_ARG, "step must be in 0..2^32-1");
+    REQUIRE(h->T > 0 && h->T < ((int64_t)1 << 32), YUE_E_UNSUPPORTED, "the log must hold 1..2^32-1 training events");
+    if (int rc = ensure_ev_user(h)) return rc;
+    const int64_t N = (int64_t)batch * negatives;
+    CK(h->tmp_i.resize((size_t)batch)); CK(h->tmp_j.resize((size_t)N));
+    BprAdamParams p = bpr_adam_params(h, batch, negatives, 0.0);
+    p.seed = seed; p.epoch = (uint32_t)step;
+    bpr_adam_sample_kernel<<<(unsigned)std::min<int64_t>((N + 255) / 256, (int64_t)h->sm_count * 16), 256, 0, h->stream>>>(p, h->tmp_i.p, h->tmp_j.p);
+    ++h->launches;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(events_out, h->tmp_i.p, batch * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(neg_out, h->tmp_j.p, N * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return YUE_OK;
+}
+
+int yue_bpr_adam_steps(yue_t* h, int batch, int negatives, double lr, double reg, uint64_t seed, int64_t step_begin,
+                       int64_t step_end, double* loss_out) {
+    if (int rc = bpr_adam_check(h, batch, negatives)) return rc;
+    REQUIRE(step_begin >= 0 && step_begin <= step_end && step_end <= (int64_t)UINT32_MAX + 1, YUE_E_ARG, "step range must lie in 0..2^32");
+    REQUIRE(h->T > 0 && h->T < ((int64_t)1 << 32), YUE_E_UNSUPPORTED, "the log must hold 1..2^32-1 training events");
+    if (step_begin == step_end) return YUE_OK;
+    if (int rc = ensure_ev_user(h)) return rc;
+    if (int rc = bpr_adam_buffers(h, batch, negatives)) return rc;
+    const int64_t steps = step_end - step_begin;
+    CK(h->ba_loss.resize((size_t)steps));
+    BprAdamParams p = bpr_adam_params(h, batch, negatives, reg);
+    p.seed = seed;
+    for (int64_t s = 0; s < steps; ++s) {
+        p.epoch = (uint32_t)(step_begin + s);
+        p.loss_out = h->ba_loss.p + s;
+        if (int rc = bpr_adam_step(h, p, lr)) return rc;
+    }
+    return bpr_adam_finish(h, steps, loss_out);
+}
+
+int yue_bpr_adam_apply(yue_t* h, int64_t B, const int32_t* u, const int32_t* i, const int32_t* j, double lr, double reg,
+                       double* loss_out) {
+    if (int rc = bpr_adam_check(h, B, 1)) return rc;
+    REQUIRE(u && i && j, YUE_E_ARG, "null argument");
+    for (int64_t b = 0; b < B; ++b)
+        REQUIRE(u[b] >= 0 && u[b] < h->m && i[b] >= 0 && i[b] < h->n && j[b] >= 0 && j[b] < h->n, YUE_E_ARG, "triplet " + std::to_string(b) + ": id out of range");
+    if (int rc = bpr_adam_buffers(h, B, 1)) return rc;
+    CK(h->ba_fix.resize(3 * (size_t)B));
+    int32_t* du = h->ba_fix.p;
+    CK(cudaMemcpyAsync(du, u, B * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(du + B, i, B * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(du + 2 * B, j, B * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+    CK(h->ba_loss.resize(1));
+    BprAdamParams p = bpr_adam_params(h, B, 1, reg);
+    p.fix_u = du; p.fix_i = du + B; p.fix_j = du + 2 * B;
+    p.loss_out = h->ba_loss.p;
+    if (int rc = bpr_adam_step(h, p, lr)) return rc;
+    double loss = 0.0;
+    if (int rc = bpr_adam_finish(h, 1, &loss)) return rc;
+    if (loss_out) *loss_out = loss;
+    return YUE_OK;
+}
+
+int yue_bpr_adam_moments(yue_t* h, float* m_users, float* m_tracks, float* v_users, float* v_tracks, int64_t* steps) {
+    REQUIRE(h && h->have_factors, YUE_E_STATE, "factors not set");
+    CK(cudaSetDevice(h->device));
+    const size_t k = (size_t)h->k, ld = (size_t)h->ld, M = (size_t)(h->m + h->n);
+    if (steps) *steps = h->ba_t;
+    const bool have = h->ba_t > 0 && h->ba_am.n >= M * ld;
+    struct { float* dst; const float* src; int64_t rows; } parts[4] = {
+        {m_users, h->ba_am.p, h->m}, {m_tracks, have ? h->ba_am.p + (size_t)h->m * ld : nullptr, h->n},
+        {v_users, h->ba_av.p, h->m}, {v_tracks, have ? h->ba_av.p + (size_t)h->m * ld : nullptr, h->n}};
     for (auto& x : parts) {
         if (!x.dst || x.rows == 0) continue;
         if (!have) { std::memset(x.dst, 0, (size_t)x.rows * k * sizeof(float)); continue; }

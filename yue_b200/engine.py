@@ -244,6 +244,40 @@ class Engine:
                                           C.byref(steps)))
         return mu, mt, vu, vt, steps.value
 
+    # ---- BPR's shipped Adam training (K10, csrc/bpr_adam.cuh) ----
+    def bpr_adam_sample(self, seed, step, batch=512, negatives=100):
+        """The batch of step `step`: (events[batch] into the event CSR, negatives[batch, negatives]) -- check hook."""
+        ev, neg = np.empty(int(batch), np.int32), np.empty((int(batch), int(negatives)), np.int32)
+        self._ck(self.lib.yue_bpr_adam_sample(self.h, int(seed), int(step), int(batch), int(negatives), _ptr(ev, C.c_int32),
+                                              _ptr(neg, C.c_int32)))
+        return ev, neg
+
+    def bpr_adam_steps(self, batch, negatives, lr, reg, seed, step_begin, step_end, want_loss=True):
+        """Adam steps [step_begin, step_end) on sampled batch x negatives triplets; returns the per-step losses."""
+        loss = np.zeros(max(int(step_end) - int(step_begin), 0), dtype=np.float64)
+        self._ck(self.lib.yue_bpr_adam_steps(self.h, int(batch), int(negatives), float(lr), float(reg), int(seed), int(step_begin),
+                                             int(step_end), _ptr(loss, C.c_double) if want_loss else None))
+        return loss if want_loss else None
+
+    def bpr_adam_apply(self, u, i, j, lr, reg):
+        """One Adam step on the caller's triplets (parity hook); returns the loss."""
+        u, i, j = _as(u, np.int32), _as(i, np.int32), _as(j, np.int32)
+        if not (u.shape == i.shape == j.shape) or u.ndim != 1:
+            raise ValueError("u / i / j must be equally long vectors")
+        loss = C.c_double(0.0)
+        self._ck(self.lib.yue_bpr_adam_apply(self.h, len(u), _ptr(u, C.c_int32), _ptr(i, C.c_int32), _ptr(j, C.c_int32),
+                                             float(lr), float(reg), C.byref(loss)))
+        return loss.value
+
+    def bpr_adam_moments(self):
+        """Adam's state of this path: (m_users, m_tracks, v_users, v_tracks, steps taken since set_factors)."""
+        mu, vu = np.empty((self.m, self.k), np.float32), np.empty((self.m, self.k), np.float32)
+        mt, vt = np.empty((self.n, self.k), np.float32), np.empty((self.n, self.k), np.float32)
+        steps = C.c_int64(0)
+        self._ck(self.lib.yue_bpr_adam_moments(self.h, _ptr(mu, C.c_float), _ptr(mt, C.c_float), _ptr(vu, C.c_float),
+                                               _ptr(vt, C.c_float), C.byref(steps)))
+        return mu, mt, vu, vt, steps.value
+
     def wrmf_sweep(self, side, reg, alpha=10.0, want_loss=False):
         """One WRMF half-sweep (0: every user row from the track table, 1: every track row from the user table)."""
         loss = C.c_double(0.0)
