@@ -308,7 +308,8 @@ int yue_allreduce_q_delta(yue_t* h);   /* pack + ncclAllReduce(sum, fp32) + appl
  *   yue_hot_share       tables[r] = rank r's table as a device pointer valid in this process (tables[rank] may be NULL);
  *                       moves the rows this rank owns from Q into its table; from here on yue_bpr_epoch(_part) /
  *                       yue_apr_epoch(_part) in YUE_MODE_HOGWILD work on the shared tables and Q's hot rows are STALE.
- *                       Barrier between the ranks before the first epoch call.
+ *                       Barrier between the ranks before the first epoch call.  After such an epoch yue_rank_topn,
+ *                       yue_predict and yue_get_factors (with Q) return YUE_E_STATE until the next yue_hot_pull.
  *   yue_hot_pull        copy every hot row from its owner's table into this handle's Q (ranks quiescent: sync + barrier
  *                       before, barrier after if anyone goes on training)
  *   yue_hot_unshare     yue_hot_pull, then back to the per-launch private table

@@ -50,6 +50,19 @@ def scores_fma32(P_rows, Q):
     return acc
 
 
+def tf32_trunc(x):
+    """float32 -> tf32 by truncation: the low 13 of the 23 mantissa bits cleared."""
+    b = np.ascontiguousarray(x, dtype=np.float32).view(np.uint32)
+    return (b & np.uint32(0xFFFFE000)).view(np.float32)
+
+
+def tf32_rn(x):
+    """float32 -> tf32 rounded to nearest, ties to even, at mantissa bit 13 (finite inputs)."""
+    b = np.ascontiguousarray(x, dtype=np.float32).view(np.uint32).astype(np.uint64)
+    b = (b + 0xFFF + ((b >> 13) & 1)) & 0xFFFFE000
+    return b.astype(np.uint32).view(np.float32)
+
+
 def topn_exact(P, Q, users, N, uq_indptr, uq_items, scores=None):
     """ids [B,N] int32 (-1 padded), scores [B,N] float32 (-inf padded)."""
     users = np.asarray(users, dtype=np.int64)

@@ -59,9 +59,15 @@ def test_device_metrics_edge_cases(engine):
     assert (ids < 0).any()
     sums, distinct = engine.rank_metrics([10, 40])
     origin = [log.test_items[log.test_indptr[u]:log.test_indptr[u + 1]].tolist() for u in users]
+    ne = [b for b, o in enumerate(origin) if len(o)]                # an empty test row adds 0 to every sum on the device
+    assert len(ne) < len(origin)
     for k, n in enumerate((10, 40)):
         rec = [[t for t in row[:n] if t >= 0] for row in ids.tolist()]
         assert sums[k, 0] == sum(metrics.hits(origin, rec))
         assert distinct[k] == len(set(t for r in rec for t in r))
+        o_ne, r_ne = [origin[b] for b in ne], [rec[b] for b in ne]
+        assert sums[k, 1] == pytest.approx(metrics.recall(metrics.hits(o_ne, r_ne), o_ne) * len(ne), rel=1e-12)
+        assert sums[k, 2] == pytest.approx(metrics.mean_ap(o_ne, r_ne, n) * len(ne), rel=1e-12)
+        assert sums[k, 3] == pytest.approx(metrics.ndcg(o_ne, r_ne, n) * len(ne), rel=1e-12)
     with pytest.raises(YueError):
         engine.rank_metrics([41])                                  # beyond the N of the last ranking call

@@ -203,7 +203,10 @@ def test_exact_kernel_catalog_split_and_stats(engine):
         ids, sc = engine.rank_topn(users, N, RANK_EXACT)
         rid, rsc = topn.topn_exact(P, Q, users, N, indptr, uq)
         assert np.array_equal(ids, rid) and np.array_equal(sc, rsc)
-    engine.rank_topn(np.arange(m, dtype=np.int32).repeat(8), 10, RANK_TC)
+    rep = np.arange(m, dtype=np.int32).repeat(8)        # every user eight times in one batch
+    ids, sc = engine.rank_topn(rep, 10, RANK_TC)
+    rid, rsc = topn.topn_exact(P, Q, rep, 10, indptr, uq)
+    assert np.array_equal(ids, rid) and np.array_equal(sc, rsc)
     fb, spilled = engine.rank_stats()
     assert fb >= 0 and spilled >= 0
 

@@ -253,6 +253,7 @@ struct yue_handle {
 
     // multi-GPU, shared hot rows (yue_hot_share) and the overlapped exchange of the tail (yue_q_exchange_*)
     bool hot_shared = false;
+    bool hot_stale = false;                   // a shared epoch trained the owners' rows: Q's copies wait for yue_hot_pull
     int hot_nranks = 1, hot_rank = 0;
     DevBuf<unsigned long long> hot_base;      // [n_hot] this process's address of the table that owns each slot
     std::vector<void*> ipc_opened;            // peer tables mapped by yue_hot_table_open ...
@@ -618,6 +619,7 @@ static int finish_interactions(yue_t* h, const int64_t* ev_indptr, const int64_t
     h->n_hot = 0;
     h->h_hot_items.clear();
     h->hot_shared = false;                     // a new log: its hot set is private until yue_hot_share is called again
+    h->hot_stale = false;
     if (T > 0 && h->hot_max > 0) {
         CK(h->item_counts.resize(n));
         CK(cudaMemsetAsync(h->item_counts.p, 0, n * sizeof(int32_t), h->stream));
@@ -862,6 +864,7 @@ int yue_set_factors(yue_t* h, int k, const float* P, const float* Q) {
     h->have_snap = false;
     h->exchange_pending = false;
     h->hot_shared = false;                     // new tables: the owners' rows no longer describe them
+    h->hot_stale = false;
     h->tc.q_dirty = true;
     h->rowmajor_current = true;
     h->ilv_current = false;
@@ -870,6 +873,7 @@ int yue_set_factors(yue_t* h, int k, const float* P, const float* Q) {
 
 int yue_get_factors(yue_t* h, float* P, float* Q) {
     REQUIRE(h && h->have_factors, YUE_E_STATE, "factors not set");
+    if (Q) REQUIRE(!h->hot_stale, YUE_E_STATE, "the shared hot rows were trained since the last yue_hot_pull: Q holds stale copies of them");
     CK(cudaSetDevice(h->device));
     if (Q) { if (int rc = q_rowmajor(h)) return rc; }
     const int k = h->k, ld = h->ld;
@@ -1113,6 +1117,7 @@ static int run_sgd(yue_t* h, SgdParams sp, int mode, double* loss_out, bool apr 
     }
     if (ilv) h->rowmajor_current = false; else h->ilv_current = false;   // the other copy is stale now
     h->tc.q_dirty = true;
+    if (blk && h->hot_shared && sp.n_hot > 0) h->hot_stale = true;      // the hot rows were trained in the owners' tables
     if (loss_out) {
         CK(cudaMemcpyAsync(loss_out, h->scal.p, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
@@ -1788,6 +1793,7 @@ int yue_frob2(yue_t* h, double* p2, double* q2) {
 int yue_predict(yue_t* h, int64_t user, float* scores_out) {
     REQUIRE(h && h->have_factors, YUE_E_STATE, "factors not set");
     REQUIRE(user >= 0 && user < h->m && scores_out, YUE_E_ARG, "bad user or null output");
+    REQUIRE(!h->hot_stale, YUE_E_STATE, "the shared hot rows were trained since the last yue_hot_pull: Q holds stale copies of them");
     CK(cudaSetDevice(h->device));
     if (int rc = q_rowmajor(h)) return rc;
     CK(h->pred.resize(h->n));
@@ -1840,6 +1846,7 @@ int yue_rank_topn(yue_t* h, const int32_t* users, int64_t B, int N, int algo, in
     REQUIRE(B >= 0 && (B == 0 || (users && ids_out && scores_out)), YUE_E_ARG, "null argument");
     REQUIRE(N >= 1 && N <= 128, YUE_E_ARG, "N must be in 1..128 (the reference caps it at 100)");
     REQUIRE(algo >= YUE_RANK_EXACT && algo <= YUE_RANK_AUTO, YUE_E_ARG, "unknown algo");
+    REQUIRE(!h->hot_stale, YUE_E_STATE, "the shared hot rows were trained since the last yue_hot_pull: Q holds stale copies of them");
     for (int64_t b = 0; b < B; ++b) REQUIRE(users[b] >= 0 && users[b] < h->m, YUE_E_ARG, "user index out of range");
     CK(cudaSetDevice(h->device));
     if (B == 0) return YUE_OK;
@@ -2329,6 +2336,7 @@ int yue_hot_pull(yue_t* h) {
         h->tc.q_dirty = true;
     }
     CK(cudaStreamSynchronize(h->stream));
+    h->hot_stale = false;
     return YUE_OK;
 }
 
