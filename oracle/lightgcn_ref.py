@@ -68,13 +68,18 @@ def init_tables(m, n, k, seed):
     return draw((m, k)), draw((n, k))
 
 
-def propagate(A, E0, n_layers=3):
-    """LightGCN.py:37-45.  Returns F and what the backward pass needs: the layers and their 1/norm."""
+def propagate(A, E0, n_layers=3, dtype=np.float64):
+    """LightGCN.py:37-45.  Returns F and what the backward pass needs: the layers and their 1/norm.
+
+    dtype=np.float32 runs every operation in float32 (A's values too; scipy's sparse product accumulates in the matrix's
+    type, in the order the CSR stores a row's neighbours): a second rounding of the same arithmetic, used only to calibrate
+    the tolerances the float32 kernel is held to."""
+    A, E0 = A.astype(dtype), np.asarray(E0).astype(dtype)
     layers, rinv = [E0], [None]
     F = E0.copy()
     for _ in range(n_layers):
         E = A @ layers[-1]
-        r = 1.0 / np.sqrt(np.maximum((E * E).sum(1), EPS_NORM))
+        r = (1.0 / np.sqrt(np.maximum((E * E).sum(1), dtype(EPS_NORM)))).astype(dtype)
         layers.append(E)
         rinv.append(r)
         F += E * r[:, None]
@@ -88,15 +93,17 @@ def loss_of(A, E0, m, u, i, j, reg, n_layers=3):
     return float(np.logaddexp(0.0, -y).sum() + 0.5 * reg * ((Fu * Fu).sum() + (Fi * Fi).sum() + (Fj * Fj).sum()))
 
 
-def loss_and_grad(A, E0, m, u, i, j, reg, n_layers=3):
-    """Loss of one batch and d loss / d E0 ([m+n, k], dense)."""
+def loss_and_grad(A, E0, m, u, i, j, reg, n_layers=3, dtype=np.float64):
+    """Loss of one batch and d loss / d E0 ([m+n, k], dense).  dtype: as in propagate()."""
     u, i, j = (np.asarray(x, dtype=np.int64) for x in (u, i, j))
-    F, layers, rinv = propagate(A, E0, n_layers)
+    A = A.astype(dtype)
+    F, layers, rinv = propagate(A, E0, n_layers, dtype)
+    reg = dtype(reg)
     Fu, Fi, Fj = F[u], F[m + i], F[m + j]
     y = (Fu * Fi).sum(1) - (Fu * Fj).sum(1)
     loss = float(np.logaddexp(0.0, -y).sum() + 0.5 * reg * ((Fu * Fu).sum() + (Fi * Fi).sum() + (Fj * Fj).sum()))
-    c = 1.0 / (1.0 + np.exp(y))                               # 1 - sigmoid(y)
-    G = np.zeros_like(E0)
+    c = (1.0 / (1.0 + np.exp(y))).astype(dtype)               # 1 - sigmoid(y)
+    G = np.zeros_like(F)
     np.add.at(G, u, -c[:, None] * (Fi - Fj) + reg * Fu)
     np.add.at(G, m + i, -c[:, None] * Fu + reg * Fi)
     np.add.at(G, m + j, c[:, None] * Fu + reg * Fj)
@@ -104,7 +111,7 @@ def loss_and_grad(A, E0, m, u, i, j, reg, n_layers=3):
     def norm_bwd(k):                                          # d/dE_k of l2_normalize(E_k), applied to G
         E, r = layers[k], rinv[k]
         nrm = E * r[:, None]
-        clamped = (E * E).sum(1) <= EPS_NORM
+        clamped = (E * E).sum(1) <= dtype(EPS_NORM)
         out = r[:, None] * (G - nrm * (nrm * G).sum(1)[:, None])
         out[clamped] = r[clamped, None] * G[clamped]
         return out
@@ -132,8 +139,9 @@ def batch_negatives(seed, epoch, ev_user, n, uq_indptr, uq_items):
 
 
 def train(A, U, V, ev_user, ev_item, uq_indptr, uq_items, batch_size, lr, reg, seed, epochs=1, n_layers=3, adam=None,
-          max_steps=None):
-    """LightGCN.py:81-98 in float64 on copies of U, V.  Returns U, V, the per-step losses and the Adam state."""
+          max_steps=None, dtype=np.float64):
+    """LightGCN.py:81-98 on copies of U, V (float64; dtype: as in propagate(), the gradient only).  Returns U, V, the
+    per-step losses and the Adam state."""
     m, n = U.shape[0], V.shape[0]
     E0 = np.concatenate([U, V]).astype(np.float64)
     adam = adam or Adam(E0.shape)
@@ -145,8 +153,8 @@ def train(A, U, V, ev_user, ev_item, uq_indptr, uq_items, batch_size, lr, reg, s
             if max_steps is not None and len(losses) >= max_steps:
                 break
             sl = slice(b0, min(T, b0 + batch_size))
-            loss, g = loss_and_grad(A, E0, m, ev_user[sl], ev_item[sl], neg[sl], reg, n_layers)
-            adam.step(E0, g, lr)
+            loss, g = loss_and_grad(A, E0, m, ev_user[sl], ev_item[sl], neg[sl], reg, n_layers, dtype)
+            adam.step(E0, g.astype(np.float64), lr)
             losses.append(loss)
     return E0[:m].copy(), E0[m:].copy(), np.array(losses), adam
 
@@ -155,3 +163,70 @@ def embeddings(A, U, V, n_layers=3):
     """The tables predict() ranks with (LightGCN.py:45-47, 101-105)."""
     F, _, _ = propagate(A, np.concatenate([U, V]).astype(np.float64), n_layers)
     return F[:U.shape[0]], F[U.shape[0]:]
+
+
+# ---- the kernel's work plan (csrc/yue_b200.cu gcn_plan), restated so tests can say which path an input takes ----
+HEAVY = 64                      # kGcnHeavy: a row with more neighbours is cut into chunks
+SEG_ROWS, SEG_EDGES = 8, 64     # kGcnSegRows, kGcnSegEdges
+HASH_SIZE = 8192                # kGcnHashSize
+SMEM_SLOTS = 3072               # kGcnSmemSlots: batches of more than 1024 triplets keep their slot list in global memory
+PAD_CHUNK = 0x7fffffff          # n_chunks of the empty chunks that pad the list to a multiple of 4
+
+
+def gcn_hash(r):
+    """The bucket of graph row r in the stamped rows' shared-memory hash (lightgcn.cuh gcn_hash): Fibonacci hashing, 13 bits."""
+    return ((int(r) * 2654435761) & 0xFFFFFFFF) >> 19
+
+
+def plan(m, n, uq_indptr, it_indptr):
+    """gcn_plan's rules.  Graph rows are users 0..m-1, then tracks m..m+n-1; a row's degree is its number of distinct
+    neighbours.  Returns (segs, heavy, chunks):
+      segs    [(first row, rows)]: runs of consecutive rows with at most HEAVY neighbours each, at most SEG_ROWS rows and
+              SEG_EDGES neighbours together, never across row m; sorted by neighbours, most first (stable)
+      heavy   the rows with more than HEAVY neighbours, most first (stable)
+      chunks  [(row, off, len, slot, first_slot, n_chunks, hidx)]: heavy row hidx cut into chunks of
+              max(ceil(sqrt(deg) / 8) * 8, HEAVY) neighbours, then empty chunks (row 0, n_chunks PAD_CHUNK, hidx = len(heavy))
+              up to a multiple of 4
+    This is a description of the plan for tests to assert which path an input takes, not a second implementation."""
+    uq_indptr, it_indptr = np.asarray(uq_indptr, np.int64), np.asarray(it_indptr, np.int64)
+    deg = np.concatenate([np.diff(uq_indptr), np.diff(it_indptr)])
+    segs, heavy = [], []
+    open_row, open_edges = -1, 0
+
+    def close(r):
+        nonlocal open_row, open_edges
+        if open_row >= 0:
+            segs.append((open_row, r - open_row))
+        open_row, open_edges = -1, 0
+    for r in range(m + n):
+        d = int(deg[r])
+        if r == m:
+            close(r)
+        if d > HEAVY:
+            close(r)
+            heavy.append(r)
+            continue
+        if open_row >= 0 and (r - open_row >= SEG_ROWS or open_edges + d > SEG_EDGES):
+            close(r)
+        if open_row < 0:
+            open_row = r
+        open_edges += d
+    close(m + n)
+    segs.sort(key=lambda sg: -int(deg[sg[0]:sg[0] + sg[1]].sum()))
+    heavy.sort(key=lambda r: -int(deg[r]))
+    chunks = []
+    for hi, r in enumerate(heavy):
+        d = int(deg[r])
+        c = max(int(np.ceil(np.sqrt(d) / 8.0)) * 8, HEAVY)
+        nck, first = (d + c - 1) // c, len(chunks)
+        chunks += [(r, q * c, min(c, d - q * c), first + q, first, nck, hi) for q in range(nck)]
+    while len(chunks) % 4:
+        chunks.append((0, 0, 0, len(chunks), len(chunks), PAD_CHUNK, len(heavy)))
+    return segs, heavy, chunks
+
+
+def degrees(m, n, uq_indptr, uq_items):
+    """Distinct neighbours of every graph row (users, then tracks) and the track side's indptr."""
+    it_indptr = np.zeros(n + 1, np.int64)
+    np.cumsum(np.bincount(np.asarray(uq_items), minlength=n), out=it_indptr[1:])
+    return np.concatenate([np.diff(np.asarray(uq_indptr, np.int64)), np.diff(it_indptr)]), it_indptr
